@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — genomic positions/sec to bedMethyl for the `modkit pileup` hot path on B200 (strong scaling).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...      (N > 1, one rank per GPU)
 
 Workload (config.workload): ONE fixed synthetic genome for every N (strong scaling) — 8 contigs, 515,553,336 bp in total
@@ -19,6 +19,9 @@ mkp_fetch_rows (== mkp_pileup_chunk) on pinned HOST buffers, copies inside the t
 with the CPU restatement's bedMethyl of a window (`parity_checked_rows`).
 `--impl reference` times the CPU restatement of the reference (oracle/, the Rust crate cannot be built here) on a bounded
 window of the same genome with every host core.
+`--dump-outputs DIR` writes what the timed path computed in its last step (see output_arrays) as DIR/<name>.npy; the genome is
+generated from a fixed seed, so two builds run with the same arguments can be compared output for output.
+bench.py compiles nothing and writes nothing under the tree (which may be read-only): it uses what build() left there.
 """
 import argparse
 import ctypes
@@ -44,6 +47,8 @@ INTERVAL = 100_000
 CPU_WINDOW = 48_000_000                # bounded CPU sample: first 48 Mb of contig 1 (480 intervals of 100 kb)
 E2E_SUB_BP = 8_000_000                 # e2e: sub-chunks pipelined over two contexts
 PRESET = ["--preset", "traditional"]
+DUMP_ROWS = 500_000                    # --dump-outputs: sampled rows of the last step (13 float64 arrays: 52 MB)
+ROW_FIELDS = ["pos", "code", "strand", "primary_base", "n_mod", "n_canon", "n_other", "n_delete", "n_filtered", "n_diff", "n_nocall"]
 
 
 def genome(scale=1.0):
@@ -57,9 +62,12 @@ def sh(cmd, **kw):
 
 
 def ensure_tools():
-    import __graft_entry__ as ge
-    ge.build_native()
-    return (os.path.join(ROOT, "tools", "_build", "synth_modbam"), os.path.join(ROOT, "oracle", "_build", "modkit_oracle"))
+    """The genome generator and the CPU oracle as build() left them."""
+    tools = (os.path.join(ROOT, "tools", "_build", "synth_modbam"), os.path.join(ROOT, "oracle", "_build", "modkit_oracle"))
+    missing = [p for p in tools if not os.access(p, os.X_OK)]
+    if missing:
+        raise SystemExit("bench.py: %s missing; build first (python __graft_entry__.py)" % ", ".join(missing))
+    return tools
 
 
 def shared_dir(tag):
@@ -140,6 +148,31 @@ def median(xs):
     return xs[len(xs) // 2]
 
 
+def output_arrays(pieces, rows, sample, seed):
+    """--dump-outputs: rows[i] are the rows (modkit_b200.ROW_DTYPE) a caller of the timed path receives for pieces[i] = (tid, lo, hi).
+    Returns float64 arrays (positions exceed float32's integers): a seeded sample of at most `sample` rows of the concatenated
+    output - every field, the contig and the row's index - and, for the whole output, each piece's row count and the CRC32 of its
+    rows' fields."""
+    import zlib
+    import numpy as np
+    from numpy.lib import recfunctions
+
+    counts = np.array([len(r) for r in rows], dtype=np.int64)
+    ends = np.cumsum(counts)
+    idx = np.sort(np.random.default_rng(seed).choice(int(ends[-1]), size=min(sample, int(ends[-1])), replace=False))
+    which = np.searchsorted(ends, idx, side="right")
+    local = idx - (ends - counts)[which]
+    picked = np.concatenate([r[local[which == i]] for i, r in enumerate(rows)])
+    out = {"rows_" + f: picked[f].astype(np.float64) for f in ROW_FIELDS}
+    out["rows_contig"] = np.array([p[0] for p in pieces], dtype=np.float64)[which]
+    out["rows_index"] = idx.astype(np.float64)
+    out["pieces"] = np.array(pieces, dtype=np.float64).reshape(-1, 3)
+    out["piece_rows"] = counts.astype(np.float64)
+    out["piece_crc32"] = np.array([zlib.crc32(recfunctions.repack_fields(r[ROW_FIELDS]).view(np.uint8)) for r in rows], dtype=np.float64)
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -151,7 +184,11 @@ def main():
     ap.add_argument("--keep", action="store_true")
     ap.add_argument("--workdir", default=None, help="(development) reuse/keep the generated workload in this directory")
     ap.add_argument("--skip-cpu", action="store_true", help="(development, A/B runs) leave cpu_baseline and the parity check out")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float64, at most 64 MB)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     a.warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -205,11 +242,7 @@ def main():
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    if rank == 0:
-        ensure_tools()
-    if world > 1:
-        dist.barrier()
-    synth, oracle = os.path.join(ROOT, "tools", "_build", "synth_modbam"), os.path.join(ROOT, "oracle", "_build", "modkit_oracle")
+    synth, oracle = ensure_tools()
     lib = modkit_b200.load_library(build_if_missing=False)
     # host threads and (first-touch) pinned buffers on the NUMA node of this rank's GPU
     numa = modkit_b200.bind_host_thread(local_rank)
@@ -340,6 +373,12 @@ def main():
             t_res = time.perf_counter() - t0
         stage /= a.steps
         l_res = launches() - l0
+        if a.dump_outputs:
+            # what mkp_fetch_rows hands the caller after the last timed mkp_pileup_resident (fetched outside the timed region)
+            arrays = output_arrays(mine, [cx.fetch_rows() for cx, _, _ in resident], DUMP_ROWS // world, SEED + rank)
+            os.makedirs(a.dump_outputs, exist_ok=True)
+            for name, arr in arrays.items():
+                np.save(os.path.join(a.dump_outputs, ("rank%d_" % rank if world > 1 else "") + name + ".npy"), arr)
 
         # ---- e2e: pinned host buffers -> rows on the host, every step; two contexts (two streams, two host threads) take
         # the sub-chunks alternately so that the H2D copy of one overlaps the kernels of the other. Every sub-chunk goes through
@@ -507,4 +546,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True     # no __pycache__ under the tree
     sys.exit(main())
