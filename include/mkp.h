@@ -102,13 +102,37 @@ typedef struct {          /* per-chunk counters, filled by mkp_pileup_* */
     uint32_t n_reads_skipped; /* admitted reads without usable mod info (skip_set)  */
     uint32_t n_states;        /* distinct (primary base, mod code) pairs seen       */
     uint32_t device_error;    /* 0, or MKP_DERR_* bits (also turned into an error)  */
-    float    kernel_ms[8];    /* CUDA-event ms: 0 parse 1 resolve 2 rank 3 (unused) 4 counters (k_count_bases, k_count_calls beside it) 5 rows 6 host sync/alloc 7 total */
+    float    kernel_ms[8];    /* CUDA-event ms: 0 parse 1 resolve 2 rank 3 (unused) 4 counters (k_count_bases, k_count_calls beside it) 5 rows 6 host sync/alloc 7 total
+                                 (mkp_hemi_resident: 2 column rank, 4 k_hemi_pairs, 5 k_hemi_rows + scan) */
 } mkp_stats;
 
 #define MKP_DERR_TOO_MANY_STATES   1u   /* > 32 distinct (base,code) states                      */
 #define MKP_DERR_TOO_MANY_LISTS    2u   /* > 16 MM lists in one read                             */
 #define MKP_DERR_TOO_MANY_CODES    4u   /* > 4 codes at one read position                        */
 #define MKP_DERR_IMPLICIT_MODE     8u   /* reserved (implicit '.'/default-mode fill is done on the device)      */
+#define MKP_DERR_TOO_MANY_PATTERNS 16u  /* pileup-hemi: > 256 distinct (base, top, bottom) patterns in one chunk   */
+
+/* ---- `modkit pileup-hemi` (src/pileup/duplex.rs, src/writers.rs:185-255) -------------------------------------------
+ * One row per (position, primary base, pattern) == DuplexPatternCounts; valid coverage = count + n_other_pattern, the
+ * percentage is formatted by the host. A half of the pattern is 0 for a canonical call ('-'), else a code point or
+ * 0x80000000|ChEBI as in mkp_row. primary_base is the read base (0..3 = A C G T). */
+typedef struct {
+    uint32_t pos;
+    uint8_t  primary_base;
+    uint8_t  reserved[3];
+    uint32_t top_code, bottom_code;
+    uint32_t count, n_canonical, n_other_pattern, n_delete, n_fail, n_diff, n_nocall;
+} mkp_hemi_row;           /* 44 bytes */
+
+/* The hemi pass on the resident chunk. The chunk must carry two bitmaps: focus_pos = the hemi columns (the positive-strand
+ * positions of the palindromic motif), focus_neg = their partner positions (column + offset); every partner must lie inside
+ * [start, end) of the chunk. offset = MotifInfo::offset (reverse minus forward motif offset; may be negative).
+ * interval_starts: the starts of the reference intervals the chunk covers, ascending (n_intervals >= 1, host memory): a read
+ * without usable mod info adds one NoCall per interval, at its first column there. Rows stay on the device. */
+int  mkp_hemi_resident(mkp_ctx* ctx, int32_t offset, const uint32_t* interval_starts, uint32_t n_intervals, mkp_stats* stats);
+/* Rows of the last mkp_hemi_resident (host memory owned by ctx), sorted by position, primary base, top half, bottom half
+ * (Canonical < code < ChEBI). */
+int  mkp_fetch_hemi_rows(mkp_ctx* ctx, const mkp_hemi_row** rows, size_t* n_rows);
 
 int  mkp_create(int device, mkp_ctx** out);
 /* Pin the calling host thread (threads it creates later inherit the mask) to the CPUs of the NUMA node the device hangs off,

@@ -47,15 +47,23 @@ ROW_DTYPE = np.dtype([("pos", "<u4"), ("code", "<u4"), ("strand", "u1"), ("prima
                       ("n_filtered", "<u4"), ("n_diff", "<u4"), ("n_nocall", "<u4")])
 assert ROW_DTYPE.itemsize == 40
 
+# mkp_hemi_row: one `modkit pileup-hemi` row; a half code is 0 for canonical ('-'), else a code point or 0x80000000|ChEBI
+HEMI_ROW_DTYPE = np.dtype([("pos", "<u4"), ("primary_base", "u1"), ("reserved", "u1", (3,)), ("top_code", "<u4"), ("bottom_code", "<u4"),
+                           ("count", "<u4"), ("n_canonical", "<u4"), ("n_other_pattern", "<u4"), ("n_delete", "<u4"),
+                           ("n_fail", "<u4"), ("n_diff", "<u4"), ("n_nocall", "<u4")])
+assert HEMI_ROW_DTYPE.itemsize == 44
+
 MKP_SYMBOLS = ["mkp_create", "mkp_bind_host_thread", "mkp_destroy", "mkp_last_error", "mkp_set_params", "mkp_upload_chunk", "mkp_pileup_resident",
                "mkp_fetch_rows", "mkp_pileup_chunk", "mkp_sample_histogram", "mkp_sample_summary", "mkp_algorithmic_bytes", "mkp_kernel_launches",
-               "mkp_device_memory", "mkp_bam_load", "mkp_bam_load_range", "mkp_bam_load_range_fd", "mkp_bam_records", "mkp_bam_chunk", "mkp_bam_tags", "mkp_bam_inflated", "mkp_fetch_chunk"]
+               "mkp_device_memory", "mkp_bam_load", "mkp_bam_load_range", "mkp_bam_load_range_fd", "mkp_bam_records", "mkp_bam_chunk", "mkp_bam_tags", "mkp_bam_inflated", "mkp_fetch_chunk",
+               "mkp_hemi_resident", "mkp_fetch_hemi_rows"]
 MKH_SYMBOLS = ["mkh_pileup_main", "mkh_bam_open", "mkh_bam_close", "mkh_bam_n_refs", "mkh_bam_ref_name", "mkh_bam_ref_len",
                "mkh_bam_n_mapped", "mkh_bam_n_records", "mkh_pack_region", "mkh_packed_free", "mkh_packed_n_reads",
                "mkh_packed_hdrs", "mkh_packed_heap", "mkh_packed_heap_bytes", "mkh_packed_algorithmic_bytes", "mkh_format_rows",
                "mkh_motif_focus", "mkh_bam_open_device", "mkh_device_chunk", "mkh_bam_ingest_ms", "mkh_bam_total_records",
                "mkh_f32_display", "mkh_bam_partition_key", "mkh_bam_n_ranges", "mkh_pileup_main_sharded", "mkh_shard_plan",
-               "mkh_bam_open_device_pieces", "mkh_bam_fetch", "mkh_summary_main", "mkh_sample_probs_main", "mkh_partition_key_of_cells", "mkh_bam_index_n_mapped", "mkh_pct2"]
+               "mkh_bam_open_device_pieces", "mkh_bam_fetch", "mkh_summary_main", "mkh_sample_probs_main", "mkh_partition_key_of_cells", "mkh_bam_index_n_mapped", "mkh_pct2",
+               "mkh_pileup_hemi_main"]
 
 ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.POINTER(C.c_uint64), C.c_size_t, C.c_void_p)
 
@@ -125,6 +133,9 @@ def load_library(build_if_missing=True):
     lib.mkh_bam_total_records.restype = C.c_uint64
     lib.mkh_pileup_main.argtypes = [C.c_int, C.POINTER(C.c_char_p)]
     lib.mkh_summary_main.argtypes = [C.c_int, C.POINTER(C.c_char_p)]
+    lib.mkh_pileup_hemi_main.argtypes = [C.c_int, C.POINTER(C.c_char_p)]
+    lib.mkp_hemi_resident.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_uint32, C.POINTER(Stats)]
+    lib.mkp_fetch_hemi_rows.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
     lib.mkh_sample_probs_main.argtypes = [C.c_int, C.POINTER(C.c_char_p)]
     lib.mkh_bam_open.argtypes = [C.c_char_p, C.c_int, C.POINTER(C.c_void_p)]
     lib.mkh_bam_close.argtypes = [C.c_void_p]
@@ -256,6 +267,13 @@ def summary_main(args):
     lib = load_library()
     argv = (C.c_char_p * len(args))(*[str(a).encode() for a in args])
     return lib.mkh_summary_main(len(args), argv)
+
+
+def pileup_hemi_main(args):
+    """In-process `modkit pileup-hemi <args>` (-o FILE, else stdout); returns the exit code (0 ok, 1 runtime error, 2 usage)."""
+    lib = load_library()
+    argv = (C.c_char_p * len(args))(*[str(a).encode() for a in args])
+    return lib.mkh_pileup_hemi_main(len(args), argv)
 
 
 def sample_probs_main(args):
@@ -467,6 +485,22 @@ class Context:
             return np.zeros(0, dtype=ROW_DTYPE)
         buf = (C.c_uint8 * (40 * n.value)).from_address(rows.value)
         return np.frombuffer(buf, dtype=ROW_DTYPE)   # view of ctx-owned pinned memory; copy() to keep
+
+    def hemi_resident(self, offset, interval_starts):
+        """The `pileup-hemi` pass on the resident chunk (uploaded with focus_pos = columns, focus_neg = partners)."""
+        starts = np.ascontiguousarray(interval_starts, dtype=np.uint32)
+        st = Stats()
+        self._check(self._lib.mkp_hemi_resident(self._h, int(offset), starts.ctypes.data, len(starts), C.byref(st)))
+        return st
+
+    def fetch_hemi_rows(self):
+        rows = C.c_void_p()
+        n = C.c_size_t()
+        self._check(self._lib.mkp_fetch_hemi_rows(self._h, C.byref(rows), C.byref(n)))
+        if not n.value:
+            return np.zeros(0, dtype=HEMI_ROW_DTYPE)
+        buf = (C.c_uint8 * (HEMI_ROW_DTYPE.itemsize * n.value)).from_address(rows.value)
+        return np.frombuffer(buf, dtype=HEMI_ROW_DTYPE)   # view of ctx-owned memory; copy() to keep
 
     def pileup_chunk(self, packed):
         ch = packed.chunk()

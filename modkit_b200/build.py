@@ -25,8 +25,8 @@ def build(force=False, verbose=False):
     csrc = os.path.join(HERE, "csrc")
     host = os.path.join(csrc, "host")
     inc = os.path.join(os.path.dirname(HERE), "include", "mkp.h")
-    dev_src = [os.path.join(csrc, "mkp_device.cu"), os.path.join(csrc, "mkp_kernels.cuh"), os.path.join(csrc, "mkp_ingest.cuh"), os.path.join(csrc, "mkp_fused.cuh"), os.path.join(csrc, "mkp_tile.cuh"), inc]
-    host_src = [os.path.join(host, f) for f in ("capi.cpp", "bam_reader.hpp", "pileup_host.hpp", "pileup_run.hpp")] + [inc]
+    dev_src = [os.path.join(csrc, "mkp_device.cu"), os.path.join(csrc, "mkp_kernels.cuh"), os.path.join(csrc, "mkp_ingest.cuh"), os.path.join(csrc, "mkp_fused.cuh"), os.path.join(csrc, "mkp_tile.cuh"), os.path.join(csrc, "mkp_hemi.cuh"), inc]
+    host_src = [os.path.join(host, f) for f in ("capi.cpp", "bam_reader.hpp", "pileup_host.hpp", "pileup_run.hpp", "pileup_hemi.hpp")] + [inc]
     lib = os.path.join(OUT, "libmodkit_b200.so")
     exe = os.path.join(OUT, "modkit")
     common = ["-O3", "-std=c++17", "-lineinfo", "--fmad=false", "-Xcompiler", "-fPIC,-O3,-pthread,-ffp-contract=off"]

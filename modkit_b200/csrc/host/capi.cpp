@@ -1,5 +1,5 @@
 // Host C API used by the Python mirror (modkit_b200/__init__.py), tests and bench.py.
-#include "pileup_run.hpp"
+#include "pileup_hemi.hpp"
 
 using namespace mkh;
 
@@ -15,6 +15,16 @@ int mkh_pileup_main(int argc, const char* const* argv) {
     if (!parse_pileup_args(argc, argv, &o, &err)) { fprintf(stderr, "error: %s\n", err.c_str()); return 2; }
     RunSummary s;
     if (run_pileup_devices(o, &s, &err)) { fprintf(stderr, "> Error! %s\n", err.c_str()); return 1; }
+    return 0;
+}
+
+// In-process `modkit pileup-hemi` (src/pileup/subcommand.rs:825-1514): argument errors exit 2 before any device is opened.
+int mkh_pileup_hemi_main(int argc, const char* const* argv) {
+    HemiOptions o;
+    std::string err;
+    if (!parse_hemi_args(argc, argv, &o, &err)) { fprintf(stderr, "error: %s\n", err.c_str()); return 2; }
+    RunSummary s;
+    if (run_pileup_hemi(o, &s, &err)) { fprintf(stderr, "> Error! %s\n", err.c_str()); return 1; }
     return 0;
 }
 

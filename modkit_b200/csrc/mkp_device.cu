@@ -19,6 +19,7 @@
 #include "mkp_fused.cuh"
 #include "mkp_tile.cuh"
 #include "mkp_ingest.cuh"
+#include "mkp_hemi.cuh"
 
 using namespace mkp;
 
@@ -91,7 +92,14 @@ struct mkp_ctx {
     std::vector<uint64_t> h_entry_off;
     mkp_row* h_rows_pinned = nullptr;
     size_t h_rows_pinned_cap = 0;
+    // pileup-hemi: pattern registry, interval starts, column rank, per-column counters, rows
+    DevBuf d_hemi_pat, d_hemi_iv, d_hemi_prefix, d_hemi_slots, d_hemi_rows;
+    uint32_t hemi_pat_cap = 8;
+    size_t n_hemi_rows = 0;
+    std::vector<mkp_hemi_row> h_hemi_rows;
 };
+
+static_assert(sizeof(mkp_hemi_row) == 44, "mkp_hemi_row is part of the C ABI");
 
 // d_small layout (u64 words): [0..31] states, [32] total_calls, [33] hist_inexact ; u32 view from byte 34*8: n_states, err, n_hot, n_rows
 static constexpr size_t SMALL_BYTES = 34 * 8 + 16 * 4;
@@ -170,7 +178,8 @@ void mkp_destroy(mkp_ctx* ctx) {
                       &ctx->d_calls, &ctx->d_hot, &ctx->d_hot_prefix, &ctx->d_block_sums, &ctx->d_small, &ctx->d_scr_cq, &ctx->d_scr_cr, &ctx->d_slow,
                       &ctx->d_obs_word, &ctx->d_slots, &ctx->d_row_counts, &ctx->d_row_prefix, &ctx->d_rows, &ctx->d_hist, &ctx->d_take,
                       &ctx->d_file, &ctx->d_members, &ctx->d_bam, &ctx->d_seeds, &ctx->d_seg_counts, &ctx->d_seg_base, &ctx->d_recs, &ctx->d_ids, &ctx->d_plan,
-                      &ctx->d_need, &ctx->d_totals, &ctx->d_slab_work, &ctx->d_pscr, &ctx->d_inftab, &ctx->d_tiles, &ctx->d_order};
+                      &ctx->d_need, &ctx->d_totals, &ctx->d_slab_work, &ctx->d_pscr, &ctx->d_inftab, &ctx->d_tiles, &ctx->d_order,
+                      &ctx->d_hemi_pat, &ctx->d_hemi_iv, &ctx->d_hemi_prefix, &ctx->d_hemi_slots, &ctx->d_hemi_rows};
     for (auto* b : bufs) b->release();
     if (ctx->h_rows_pinned) cudaFreeHost(ctx->h_rows_pinned);
     for (int i = 0; i < ctx->n_pin; i++) { cudaFreeHost(ctx->pin[i]); cudaEventDestroy(ctx->pin_ev[i]); }
@@ -284,6 +293,7 @@ static std::string derr_text(uint32_t e) {
     if (e & MKP_DERR_TOO_MANY_STATES) s += "more than 32 distinct (base, mod code) states; ";
     if (e & MKP_DERR_TOO_MANY_LISTS) s += "more than 16 MM lists in one read; ";
     if (e & MKP_DERR_TOO_MANY_CODES) s += "more than 4 codes in one MM list or 7 at one position; ";
+    if (e & MKP_DERR_TOO_MANY_PATTERNS) s += "more than 256 distinct (base, top, bottom) hemi patterns in one chunk; ";
     return s;
 }
 
@@ -620,6 +630,140 @@ int mkp_pileup_chunk(mkp_ctx* ctx, const mkp_chunk* ch, const mkp_row** rows, si
     if (int rc = mkp_upload_chunk(ctx, ch)) return rc;
     if (int rc = mkp_pileup_resident(ctx, stats)) return rc;
     return mkp_fetch_rows(ctx, rows, n_rows);
+}
+
+// `modkit pileup-hemi` on the resident chunk: the pileup decode (k_parse, k_resolve: every read's call records), the column rank,
+// the pair kernel, the row kernels. The per-column counters hold `hemi_pat_cap` pattern counts; a chunk that shows more patterns
+// grows the capacity and runs the pair kernel again (the decode stays).
+int mkp_hemi_resident(mkp_ctx* ctx, int32_t offset, const uint32_t* interval_starts, uint32_t n_intervals, mkp_stats* stats) {
+    if (!ctx) return -1;
+    if (!ctx->have_params) return fail(ctx, "mkp_set_params was not called");
+    if (ctx->ce <= ctx->cs) return fail(ctx, "no resident chunk");
+    if (!ctx->have_focus) return fail(ctx, "mkp_hemi_resident needs the column / partner bitmaps (focus_pos / focus_neg)");
+    if (!interval_starts || n_intervals == 0) return fail(ctx, "mkp_hemi_resident needs the interval starts of the chunk");
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    ChunkDev C;
+    const int grid = decode_grid(ctx, ctx->n_reads);
+    if (int rc = prepare_decode(ctx, &C, grid)) return rc;
+    C.list_mode = 2;                                           // every read; the hot bitmap (rank of the focus set) is not touched
+    const uint32_t n_words = ctx->n_words;
+    const uint32_t n_blk = (n_words + 1023) / 1024;
+    CK(ctx->d_block_sums.ensure((size_t)n_blk * 4 + 4));
+    CK(ctx->d_row_counts.ensure((size_t)n_words * 4 + 4));
+    CK(ctx->d_row_prefix.ensure((size_t)n_words * 4 + 4));
+    CK(ctx->d_hemi_prefix.ensure((size_t)n_words * 4 + 4));
+    CK(ctx->d_hemi_pat.ensure((HEMI_MAX_PATTERNS + 4) * 4));
+    CK(ctx->d_hemi_iv.ensure((size_t)n_intervals * 4));
+    uint32_t* pat = ctx->d_hemi_pat.as<uint32_t>();
+    uint32_t* u = (uint32_t*)(ctx->d_small.as<uint8_t>() + 34 * 8);   // n_states, err, n_cols, n_rows; u[14] pair read counter
+    // events: 0 start | 1 after parse | 2 after resolve | 3 after rank | 4 before pairs | 6 after pairs | 7 after row count+scan |
+    //         8 before emit | 9 end
+    CK(cudaEventRecord(ctx->ev[0], st));
+    CK(cudaMemcpyAsync(ctx->d_hemi_iv.p, interval_starts, (size_t)n_intervals * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(pat, 0xff, HEMI_MAX_PATTERNS * 4, st));
+    CK(cudaMemsetAsync(pat + HEMI_MAX_PATTERNS, 0, 16, st));
+    CK(cudaMemsetAsync(ctx->d_small.p, 0xff, 32 * 8, st));
+    CK(cudaMemsetAsync(ctx->d_small.as<uint8_t>() + 32 * 8, 0, SMALL_BYTES - 32 * 8, st));
+    C.mode = MODE_PILEUP;
+    ctx->launches += 1; if (ctx->n_reads) k_parse<<<grid, 128, 0, st>>>(C);
+    CK(cudaEventRecord(ctx->ev[1], st));
+    ctx->launches += 2; if (ctx->n_reads) { k_resolve<MODE_PILEUP, true><<<grid, 128, 0, st>>>(C); k_resolve<MODE_PILEUP, false><<<grid, 128, 0, st>>>(C); }
+    CK(cudaEventRecord(ctx->ev[2], st));
+    // counter slot of a column = rank of its bit in focus_pos
+    uint32_t* cols = ctx->d_focus_pos.as<uint32_t>();
+    uint32_t* col_prefix = ctx->d_hemi_prefix.as<uint32_t>();
+    ctx->launches += 3;
+    k_block_popc<<<n_blk, 1024, 0, st>>>(cols, n_words, ctx->d_block_sums.as<uint32_t>(), nullptr, nullptr);
+    k_scan_blocks<<<1, 1024, 0, st>>>(ctx->d_block_sums.as<uint32_t>(), n_blk, u + 2);
+    k_word_prefix<<<n_blk, 1024, 0, st>>>(cols, n_words, ctx->d_block_sums.as<uint32_t>(), col_prefix);
+    CK(cudaEventRecord(ctx->ev[3], st));
+    uint32_t h_small[4];
+    unsigned long long h_calls = 0;
+    CK(cudaMemcpyAsync(h_small, u, 16, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&h_calls, C.total_calls, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const uint32_t n_states = h_small[0], derr = h_small[1], n_cols = h_small[2];
+    if (derr) {
+        if (stats) { memset(stats, 0, sizeof *stats); stats->device_error = derr; }
+        return fail(ctx, "device decode error: " + derr_text(derr), -10);
+    }
+    HemiDev H;
+    H.hdrs = C.hdrs; H.heap = C.heap; H.meta = C.meta; H.calls = C.calls; H.n_reads = C.n_reads; H.cs = C.cs; H.ce = C.ce;
+    H.cols = cols; H.col_prefix = col_prefix; H.offset = offset;
+    H.iv_starts = ctx->d_hemi_iv.as<uint32_t>(); H.n_iv = n_intervals;
+    H.pat_keys = pat; H.n_pat = pat + HEMI_MAX_PATTERNS; H.work = u + 14;
+    H.order = C.order; H.combine = ctx->params.numeric_mode == 1 ? 1u : 0u;
+    const int g2 = std::max(1, std::min(ctx->sm_count * 8, (int)((ctx->n_reads + 7) / 8)));
+    uint32_t n_pat = 0;
+    float pairs_ms = 0;
+    for (;;) {
+        H.pat_cap = ctx->hemi_pat_cap;
+        H.stride = HS_PAT + H.pat_cap;
+        CK(ctx->d_hemi_slots.ensure(std::max<size_t>(1, n_cols) * H.stride * 4));
+        H.slots = ctx->d_hemi_slots.as<uint32_t>();
+        CK(cudaMemsetAsync(H.slots, 0, (size_t)n_cols * H.stride * 4, st));
+        CK(cudaMemsetAsync(u + 14, 0, 4, st));
+        CK(cudaEventRecord(ctx->ev[4], st));
+        ctx->launches += 1; if (ctx->n_reads && n_cols) k_hemi_pairs<<<g2, 256, 0, st>>>(H);
+        CK(cudaEventRecord(ctx->ev[6], st));
+        CK(cudaMemcpyAsync(&n_pat, H.n_pat, 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        float ms = 0;
+        cudaEventElapsedTime(&ms, ctx->ev[4], ctx->ev[6]);
+        pairs_ms += ms;
+        if (n_pat > (uint32_t)HEMI_MAX_PATTERNS) {
+            if (stats) { memset(stats, 0, sizeof *stats); stats->device_error = MKP_DERR_TOO_MANY_PATTERNS; }
+            return fail(ctx, "device decode error: " + derr_text(MKP_DERR_TOO_MANY_PATTERNS), -10);
+        }
+        if (n_pat <= H.pat_cap) break;
+        while (ctx->hemi_pat_cap < n_pat) ctx->hemi_pat_cap *= 2;     // more patterns than counters per column: grow, count again
+    }
+    HemiRowDev R;
+    R.cols = cols; R.col_prefix = col_prefix; R.n_words = n_words; R.cs = C.cs;
+    R.slots = H.slots; R.stride = H.stride; R.n_pat = n_pat; R.pat_keys = pat; R.states = C.states;
+    R.row_counts = ctx->d_row_counts.as<uint32_t>(); R.row_prefix = ctx->d_row_prefix.as<uint32_t>(); R.rows = nullptr;
+    const int rg = (n_words + 255) / 256;
+    CK(cudaEventRecord(ctx->ev[6], st));
+    ctx->launches += 4;
+    k_hemi_rows<false><<<rg, 256, 0, st>>>(R);
+    k_block_sum<<<n_blk, 1024, 0, st>>>(R.row_counts, n_words, ctx->d_block_sums.as<uint32_t>());
+    k_scan_blocks<<<1, 1024, 0, st>>>(ctx->d_block_sums.as<uint32_t>(), n_blk, u + 3);
+    k_value_prefix<<<n_blk, 1024, 0, st>>>(R.row_counts, n_words, ctx->d_block_sums.as<uint32_t>(), ctx->d_row_prefix.as<uint32_t>());
+    CK(cudaEventRecord(ctx->ev[7], st));
+    uint32_t n_rows = 0;
+    CK(cudaMemcpyAsync(&n_rows, u + 3, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(ctx->d_hemi_rows.ensure(std::max<size_t>(1, n_rows) * sizeof(mkp_hemi_row)));
+    R.rows = ctx->d_hemi_rows.as<mkp_hemi_row>();
+    CK(cudaEventRecord(ctx->ev[8], st));
+    ctx->launches += 1; if (n_rows) k_hemi_rows<true><<<rg, 256, 0, st>>>(R);
+    CK(cudaEventRecord(ctx->ev[9], st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    ctx->n_hemi_rows = n_rows;
+    if (stats) {
+        memset(stats, 0, sizeof *stats);
+        stats->n_rows = n_rows; stats->n_hot = n_cols; stats->n_calls = h_calls; stats->n_states = n_states;
+        auto el = [&](int a, int b) { float ms = 0; cudaEventElapsedTime(&ms, ctx->ev[a], ctx->ev[b]); return ms; };
+        stats->kernel_ms[0] = el(0, 1); stats->kernel_ms[1] = el(1, 2); stats->kernel_ms[2] = el(2, 3);
+        stats->kernel_ms[4] = pairs_ms; stats->kernel_ms[5] = el(6, 7) + el(8, 9);
+        stats->kernel_ms[7] = el(0, 9); stats->kernel_ms[6] = stats->kernel_ms[7] - (el(0, 3) + pairs_ms + stats->kernel_ms[5]);
+    }
+    return 0;
+}
+
+int mkp_fetch_hemi_rows(mkp_ctx* ctx, const mkp_hemi_row** rows, size_t* n_rows) {
+    if (!ctx || !rows || !n_rows) return -1;
+    CK(cudaSetDevice(ctx->device));
+    ctx->h_hemi_rows.resize(std::max<size_t>(1, ctx->n_hemi_rows));
+    if (ctx->n_hemi_rows) {
+        CK(cudaMemcpyAsync(ctx->h_hemi_rows.data(), ctx->d_hemi_rows.p, ctx->n_hemi_rows * sizeof(mkp_hemi_row), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    *rows = ctx->h_hemi_rows.data();
+    *n_rows = ctx->n_hemi_rows;
+    return 0;
 }
 
 int mkp_sample_histogram(mkp_ctx* ctx, int include_unaligned, const uint8_t* take, uint64_t* hist, uint8_t* contributes, uint64_t* inexact) {

@@ -7,6 +7,8 @@
 //                [--mean-len 12000] [--level 1] [--threads 8] [--combined-hm] [--implicit] [--odd-records] [--partition-tags [--long-rg]]
 //                [--start-grid G]  (read starts snapped to multiples of G: stacks of reads sharing a start, for --max-depth)
 //                [--region-only START-END]   (only reads overlapping the window; reference still full length)
+//                [--duplex]  (each read also carries G-h?/G-m? lists: calls on the opposite strand's C of every CpG, drawn
+//                             independently, so hemi-methylated patterns occur; `modkit pileup-hemi` input)
 // Writes PREFIX.fa, PREFIX.fa.fai, PREFIX.bam, PREFIX.bam.bai and prints a JSON summary (exact algorithmic bytes,
 // read-bases, reads) on stdout.
 #include <zlib.h>
@@ -50,6 +52,7 @@ struct Opts {
     bool ptags = false;    // --partition-tags: RG:Z (A/B/C or absent), HP (C or i, or absent), XF:f on some reads
     bool long_rg = false;  // --long-rg: the RG values are long run ids (ONT style, ~80 characters) ending in A/B/C
     int64_t win_start = -1, win_end = -1;
+    bool duplex = false;       // --duplex: opposite-strand CpG lists (G-h?, G-m?) beside the C+ lists
     uint32_t start_grid = 0;   // --start-grid G: read starts snapped down to multiples of G (amplicon-like stacks of reads with one start)
 };
 
@@ -184,6 +187,30 @@ static void make_read(const Opts& o, const Contig& c, int32_t tid, uint32_t star
                 else { emit(std::string("C+h") + mode, &qh, nullptr); emit(std::string("C+m") + mode, &qm, nullptr); }
             } else if (want_m) emit(std::string("C+m") + mode, &qm, nullptr);
             else emit(std::string("C+h") + mode, &qh, nullptr);
+            if (o.duplex) {
+                // the G of every CpG in read orientation: a call on the C of the opposite strand, drawn independently of the C+ call
+                std::vector<uint8_t> gh, gm;
+                deltas.clear();
+                skipped = 0;
+                for (uint32_t f = 0; f < L; f++) {
+                    if (fwd(f) != 'G') continue;
+                    if (!(f > 0 && fwd(f - 1) == 'C')) { skipped++; continue; }
+                    deltas.push_back(skipped);
+                    skipped = 0;
+                    const int64_t rp = fwd_ref(f);
+                    double level = 0.5;
+                    if (rp >= 0) { const uint32_t cpos = rev ? (uint32_t)rp : (uint32_t)rp - 1; if (cpos < c.len) level = c.meth[cpos] / 255.0; }
+                    const bool is_mod = rng.uni() < level;
+                    const bool is_h = want_h && is_mod && rng.uni() < 0.2;
+                    uint32_t qa = 225 + rng.below(31), qb = rng.below(256 - qa);
+                    if (!is_mod) { qa = rng.below(30); qb = rng.below(30); }
+                    if (want_h && want_m) { if (is_h) { gh.push_back((uint8_t)qa); gm.push_back((uint8_t)qb); } else { gm.push_back((uint8_t)qa); gh.push_back((uint8_t)qb); } }
+                    else if (want_m) gm.push_back((uint8_t)qa);
+                    else gh.push_back((uint8_t)qa);
+                }
+                if (want_h) emit(std::string("G-h") + mode, &gh, nullptr);
+                if (want_m) emit(std::string("G-m") + mode, &gm, nullptr);
+            }
         }
         if (want_a) {
             mm += std::string("A+a") + mode;
@@ -258,6 +285,7 @@ int main(int argc, char** argv) {
         else if (a == "--odd-records") o.odd = true;
         else if (a == "--partition-tags") o.ptags = true;
         else if (a == "--long-rg") o.long_rg = true;
+        else if (a == "--duplex") o.duplex = true;
         else if (a == "--start-grid") o.start_grid = (uint32_t)std::stoul(val());
         else if (a == "--region-only") { std::string s = val(); auto d = s.find('-'); o.win_start = std::stoll(s.substr(0, d)); o.win_end = std::stoll(s.substr(d + 1)); }
         else { fprintf(stderr, "unknown flag %s\n", a.c_str()); return 2; }
